@@ -2,6 +2,7 @@
 """bench.py -- throughput of the FLAC block encode/decode hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg2|cfg2_l8|cfg3|cfg4|cfg5] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch (BASELINE configs: 10 000 blocks of 4096 samples; cfg4: 125 files
 of 100 blocks per GPU). Prints ONE JSON line (rank 0). See DESIGN.md "Measurement" for the definitions:
@@ -18,8 +19,13 @@ of 100 blocks per GPU). Prints ONE JSON line (rank 0). See DESIGN.md "Measuremen
              N; the single-encoder set_num_threads(64) figure and the 1-thread figure are reported next to it.
   frames_compared / frames_equal
              every frame of the GPU stream memcmp'ed against the reference's frame for the same block, in this run.
-Without --workload the default line is cfg2 and the other BASELINE configs ride along under extra.workloads
-(fewer steps), so that one driver invocation measures all of them.
+Without --workload the default line is cfg2 and the other BASELINE configs ride along under extra.workloads,
+so that one driver invocation measures all of them. Every timed loop runs K steps.
+--dump-outputs DIR
+             after the timed steps, rank 0 writes what the last device-resident step of each workload computed to
+             DIR/<workload>_<array>.npy (float64, or float32 for bytes), so that two builds can be compared output for
+             output: the inputs depend only on the arguments. Encode: every frame offset, and the bytes of a fixed,
+             seeded sample of frames; decode: every frame status word and the samples of such a sample of frames.
 """
 import argparse
 import json
@@ -46,6 +52,9 @@ WORKLOADS = {
 DATA_NOTE = "synthetic: music-like base (SURVEY 8d-i generator) of 256 blocks tiled over the batch + independent +-1 LSB dither per sample"
 
 _pcm_cache = {}
+DUMP_FRAMES = 64          # frames per workload in the --dump-outputs sample
+DUMP_SEED = 20240601
+DUMP_LIMIT = 64 << 20     # bytes, all .npy payloads together
 
 
 def make_pcm(ch, bps, rate, blocks, bs, seed):
@@ -280,7 +289,7 @@ def run_reference_arm(args, name):
     config = config_of(name, args.gpus)
     config["blocks_per_gpu_per_step"] = blocks
     nthreads = host_threads()
-    steps = max(args.steps, 5)
+    steps = args.steps
     if name == "cfg5":
         # the reference decoder is single-threaded per stream; every host core decodes its own stream
         # (ctypes releases the GIL), as a many-file batch would
@@ -319,8 +328,21 @@ def run_reference_arm(args, name):
             "gpu_launches": 0}
 
 
+def dump_sample(blocks):
+    """The frames whose contents --dump-outputs writes: a fixed, seeded choice, the same for the same arguments."""
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(blocks, min(DUMP_FRAMES, blocks), replace=False))
+
+
+def write_dump(path, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT, f"--dump-outputs: {total} bytes exceed {DUMP_LIMIT}"
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------- B200 arm: decode
-def bench_decode(args, ranks, name, steps, warmup, with_cpu):
+def bench_decode(args, ranks, name, steps, warmup, with_cpu, dump=None):
     import ctypes as C
     import torch
     import flac_b200
@@ -388,6 +410,11 @@ def bench_decode(args, ranks, name, steps, warmup, with_cpu):
     ranks.barrier()
     dev_ms = ranks.max(ev0.elapsed_time(ev1))
     launches = dec.launches - launches0
+    if dump is not None and rank == 0:  # what the last timed step decoded: status per frame, samples of the sampled frames
+        pick = torch.from_numpy(dump_sample(blocks)).to("cuda")
+        dump[f"{name}_status"] = d_status.cpu().numpy().astype(np.float64)
+        dump[f"{name}_pcm_sample"] = d_pcm.view(blocks, bs, ch)[pick].cpu().numpy().astype(np.float64)
+        dump[f"{name}_sample_frames"] = pick.cpu().numpy().astype(np.float64)
     prof = dec.profile(reset=True)
     dec.set_profiling(False)
 
@@ -402,9 +429,9 @@ def bench_decode(args, ranks, name, steps, warmup, with_cpu):
     step_host_int32()
     ranks.barrier()
     t0 = time.perf_counter()
-    for _ in range(max(2, steps // 2)):
+    for _ in range(steps):
         step_host_int32()
-    e2e32_s = ranks.max(time.perf_counter() - t0) / max(2, steps // 2)
+    e2e32_s = ranks.max(time.perf_counter() - t0) / steps
     ranks.barrier()
     clocks = sampler.stop() if rank == 0 else None
     assert np.array_equal(h_pcm.numpy(), x), "e2e decoded PCM (int32) differs from the input"
@@ -472,7 +499,7 @@ def bench_decode(args, ranks, name, steps, warmup, with_cpu):
 
 
 # ---------------------------------------------------------------------------------------------- B200 arm: encode
-def bench_encode(args, ranks, name, steps, warmup, with_cpu):
+def bench_encode(args, ranks, name, steps, warmup, with_cpu, dump=None):
     import torch
     import flac_b200
     rank, local_rank, world = ranks.rank, ranks.local_rank, ranks.world
@@ -537,6 +564,12 @@ def bench_encode(args, ranks, name, steps, warmup, with_cpu):
     ranks.barrier()
     dev_ms = ranks.max(ev0.elapsed_time(ev1))
     launches = enc.launches - launches0
+    if dump is not None and rank == 0:  # what the last timed step encoded: every frame offset, the bytes of the sampled frames
+        offs = d_offs.cpu().numpy()
+        pick = dump_sample(blocks)
+        dump[f"{name}_offsets"] = offs.astype(np.float64)
+        dump[f"{name}_stream_sample"] = torch.cat([d_out[int(offs[i]):int(offs[i + 1])] for i in pick]).cpu().numpy().astype(np.float32)
+        dump[f"{name}_sample_frames"] = pick.astype(np.float64)
     # ---- the same K steps again with CUDA events recorded BETWEEN the kernels (per-kernel durations for the roofline; the
     # events serialise the two kernels the engine otherwise overlaps, so this pass is a little slower than the timed one)
     enc.set_profiling(True)
@@ -722,6 +755,8 @@ def main():
     ap.add_argument("--kernels-only", action="store_true", help="profiling aid: device-resident steps only (no e2e, no CPU baseline)")
     ap.add_argument("--no-extras", action="store_true", help="default invocation: only the cfg2 line, no extra.workloads")
     ap.add_argument("--full-cpu", action="store_true", help="cpu_baseline with best of 5 instead of 3")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of each workload computed to DIR/*.npy (rank 0)")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else max(args.warmup, 1)
     primary = args.workload or "cfg2"
@@ -742,25 +777,28 @@ def main():
     torch.cuda.set_device(int(os.environ.get("LOCAL_RANK", "0")))
     ranks = Ranks(backend="nccl", device="cuda")
 
+    dump = {} if args.dump_outputs else None
+
     def run(name, steps, warmup, with_cpu):
         fn = bench_decode if name == "cfg5" else bench_encode
-        return fn(args, ranks, name, steps, warmup, with_cpu)
+        return fn(args, ranks, name, steps, warmup, with_cpu, dump)
 
     line = run(primary, args.steps, args.warmup, True)
     if args.workload is None and not args.no_extras and not args.kernels_only:
         extras = {}
-        xsteps = max(3, args.steps // 4)
         for name in ("cfg2_l8", "cfg3", "cfg4", "cfg5"):
             try:
-                extras[name] = summarize(run(name, xsteps, 3, True))
+                extras[name] = summarize(run(name, args.steps, 3, True))
             except AssertionError:
                 raise
             except Exception as ex:  # an extra must never take the headline line down
                 extras[name] = {"error": f"{type(ex).__name__}: {ex}"}
         if ranks.rank == 0:
             line["extra"] = {"workloads": extras,
-                             "note": "the other BASELINE configs, same procedure, fewer timed steps; parity counted per workload"}
+                             "note": "the other BASELINE configs, same procedure; parity counted per workload"}
     if ranks.rank == 0:
+        if dump is not None:
+            write_dump(args.dump_outputs, dump)
         print(json.dumps(line))
     ranks.close()
     return 0

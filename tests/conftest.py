@@ -1,23 +1,9 @@
 import os
 import sys
 
-import pytest
-
 sys.path.insert(0, os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.abspath(os.path.join(os.path.dirname(__file__), "..")))
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: test needs a CUDA device (run on the B200 box with -m gpu)")
-
-
-@pytest.fixture(scope="session")
-def ref_available():
-    import reflib
-    return reflib.available("default") and reflib.available("strict")
-
-
-def require_ref(variant=None):
-    import reflib
-    if not (reflib.available("default") and reflib.available("strict")):
-        pytest.skip("oracle/_ref not built (run `make -C oracle ref` where /root/reference exists)")

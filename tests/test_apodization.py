@@ -3,17 +3,15 @@
 
 CPU (-m "not gpu"): the oracle's and the engine's host-side window tables against the compiled
 reference's FLAC__window_* symbols, bit for bit; oracle frames against reference frames for
-specification strings.  GPU: CUDA frames against the oracle and the compiled reference."""
-import ctypes as C
-import os
-
+specification strings.  GPU: CUDA frames against the oracle and the compiled reference.
+The reference's tables and frames are its answers stored in tests/golden/reference.json.gz (tests/refdata.py)."""
 import numpy as np
 import pytest
 
 import oraclelib
+import refdata
 import reflib
 import signals
-from conftest import require_ref
 
 # (our type id, reference symbol, extra float args)
 PLAIN = [
@@ -38,16 +36,6 @@ SPECS = [
 ]
 
 
-def _ref_window(L, sym, n, *params):
-    f = getattr(L, sym)
-    f.restype = None
-    f.argtypes = [C.c_void_p, C.c_int32] + [C.c_float] * len(params)
-    out = np.full(n + 8, np.float32(-77.0))
-    f(out.ctypes.data, n, *params)
-    assert np.all(out[n:] == np.float32(-77.0))
-    return out[:n]
-
-
 # The shipped build flags (-fassociative-math ..., oracle/Makefile REF_FAST) let GCC re-associate the
 # three-or-more-term float sums of these six generators: their tables differ from source order by
 # <= 3 ulp there (measured below).  Source order (the strict build) is the semantics we pin; the other
@@ -59,8 +47,14 @@ def _reassociated(name):
     return any(name == "FLAC__window_" + r or name == "FLAC__window_" + r + "_sidelobe" or r in name.split(";") for r in REASSOCIATED_BY_SHIPPED_FLAGS)
 
 
-def _same_bits(a, b):
-    return np.array_equal(a.view(np.uint32), b.view(np.uint32))
+def _check_window(got, variant, sym, n, params):
+    """got bit for bit the reference's table; for a re-associated generator under the shipped build, within 3 ulp(1.0)
+    of its table (checked as: bit for bit the source-order table, which lies that close to the shipped one)."""
+    if variant == "default" and _reassociated(sym):
+        assert refdata.digest(got) == refdata.window("strict", sym, n, *params)["sha"], f"{sym}{params} L={n}: not the source-order table"
+        assert refdata.window("default", sym, n, *params)["max_abs_diff_vs_strict"] <= 3 * 2.0 ** -24, f"{sym} L={n}: more than 3 ulp(1.0) from the shipped build"
+        return
+    assert refdata.digest(got) == refdata.window(variant, sym, n, *params)["sha"], f"{sym}{params} L={n} [{variant}]"
 
 
 def _window_cases():
@@ -86,32 +80,18 @@ def _apod(cls, t, params):
 
 @pytest.mark.parametrize("variant", ["strict", "default"])
 def test_oracle_window_tables_match_reference(variant):
-    require_ref(variant)
-    L = reflib.lib(variant)
     for t, sym, params in _window_cases():
         for n in LENGTHS:
-            want = _ref_window(L, sym, n, *params)
-            got = oraclelib.window(_apod(oraclelib.Apod, t, params), n)
-            if variant == "default" and _reassociated(sym):
-                assert np.abs(got - want).max() <= 3 * 2.0 ** -24, f"{sym} L={n}: more than 3 ulp(1.0) from the shipped build"
-                continue
-            assert _same_bits(got, want), f"{sym}{params} L={n} [{variant}]: {np.flatnonzero(got != want)[:5]}"
+            _check_window(oraclelib.window(_apod(oraclelib.Apod, t, params), n), variant, sym, n, params)
 
 
 @pytest.mark.parametrize("variant", ["strict", "default"])
 def test_engine_window_tables_match_reference(variant):
     """The product's host-side generators (flac_b200/csrc/windows.h via fb200_window; no GPU needed)."""
-    require_ref(variant)
     import flac_b200
-    L = reflib.lib(variant)
     for t, sym, params in _window_cases():
         for n in LENGTHS:
-            want = _ref_window(L, sym, n, *params)
-            got = flac_b200.window(_apod(flac_b200.Apodization, t, params), n)
-            if variant == "default" and _reassociated(sym):
-                assert np.abs(got - want).max() <= 3 * 2.0 ** -24, f"{sym} L={n}"
-                continue
-            assert _same_bits(got, want), f"{sym}{params} L={n} [{variant}]"
+            _check_window(flac_b200.window(_apod(flac_b200.Apodization, t, params), n), variant, sym, n, params)
 
 
 def test_engine_and_oracle_parse_specifications_identically():
@@ -133,28 +113,25 @@ def test_engine_and_oracle_parse_specifications_identically():
 
 @pytest.mark.parametrize("spec", SPECS)
 def test_oracle_frames_match_reference_for_specification(spec):
-    require_ref("strict")
     x = signals.music_like(4096 * 2 + 321, 2, 16, 44100, seed=23)
     for level, variant in ((5, "strict"), (8, "strict"), (5, "default")):
         if variant == "default" and _reassociated(spec):
             continue  # G2 is not gated where the shipped flags re-associate the window sum (see above)
         enc = oraclelib.Encoder(oraclelib.preset(2, 16, 44100, level, apodization=spec))
         got = enc.encode_stream(x)
-        _, _, ref = reflib.encode(x, 16, rate=44100, level=level, variant=variant, opts=reflib.RefEncOpts(apodization=spec))
-        assert len(got) == len(ref)
-        bad = [i for i, (a, b) in enumerate(zip(got, ref)) if a != b]
+        ref = refdata.encode(x, 16, rate=44100, level=level, variant=variant, opts=reflib.RefEncOpts(apodization=spec))
+        bad = ref.mismatches(got)
         assert not bad, f"{spec!r} level {level} [{variant}]: frames {bad} differ"
 
 
 @pytest.mark.parametrize("bs,ch,bps", [(1152, 1, 16), (4608, 2, 24), (577, 2, 16)])
 def test_oracle_frames_match_reference_other_shapes(bs, ch, bps):
-    require_ref("strict")
     x = signals.music_like(bs * 2 + 50, ch, bps, 48000, seed=29)
     for spec in ("tukey(0.25);partial_tukey(2);punchout_tukey(3)", "gauss(0.15);flattop;welch"):
         enc = oraclelib.Encoder(oraclelib.preset(ch, bps, 48000, 8, bs, apodization=spec))
         got = enc.encode_stream(x)
-        _, _, ref = reflib.encode(x, bps, rate=48000, level=8, blocksize=bs, variant="strict", opts=reflib.RefEncOpts(apodization=spec))
-        assert got == ref, spec
+        ref = refdata.encode(x, bps, rate=48000, level=8, blocksize=bs, variant="strict", opts=reflib.RefEncOpts(apodization=spec))
+        assert ref.mismatches(got) == [], spec
 
 
 # --------------------------------------------------------------------------------- GPU
@@ -169,12 +146,11 @@ def test_gpu_frames_for_specification(spec):
         enc.close()
         want = oraclelib.Encoder(oraclelib.preset(2, 16, 44100, level, apodization=spec)).encode_stream(x)
         assert got == want, f"oracle: {spec!r} level {level}"
-        if reflib.available("strict"):
-            for variant in ("strict", "default"):
-                if variant == "default" and _reassociated(spec):
-                    continue
-                _, _, ref = reflib.encode(x, 16, rate=44100, level=level, variant=variant, opts=reflib.RefEncOpts(apodization=spec))
-                assert got == ref, f"reference[{variant}]: {spec!r} level {level}"
+        for variant in ("strict", "default"):
+            if variant == "default" and _reassociated(spec):
+                continue
+            ref = refdata.encode(x, 16, rate=44100, level=level, variant=variant, opts=reflib.RefEncOpts(apodization=spec))
+            assert ref.mismatches(got) == [], f"reference[{variant}]: {spec!r} level {level}"
 
 
 @pytest.mark.gpu

@@ -1,13 +1,14 @@
 """The drop-in boundary, checked with the reference's OWN client code.
 
-CPU (this container, where /root/reference exists): the unmodified examples/c/{decode,encode}/file/main.c compile against the
-reference's headers and LINK against libflac_b200.so (every symbol they use is exported); the structs a client reads through
-the callbacks (FLAC__Frame, FLAC__StreamMetadata, ...) have the reference's layout.
-GPU: the prebuilt example binaries (oracle/_ref/examples, built by `make -C oracle examples`) run against libflac_b200.so and
-produce what the same binaries produce with the compiled reference."""
+CPU: the unmodified examples/c/{decode,encode}/file/main.c link against libflac_b200.so (every libFLAC symbol they take from
+the library is exported); the structs a client reads through the callbacks (FLAC__Frame, FLAC__StreamMetadata, ...) have the
+reference's layout. Both compare with what the reference's sources give, stored in tests/golden/dropin.json by
+tests/golden/make_dropin_golden.py.
+GPU: the prebuilt example binaries (oracle/_ref/examples, built by `make -C oracle examples` where the reference's sources
+are) run against libflac_b200.so and produce what the same binaries produce with the compiled reference."""
+import json
 import os
 import shutil
-import struct
 import subprocess
 import sys
 import wave
@@ -16,9 +17,10 @@ import numpy as np
 import pytest
 
 ROOT = os.path.abspath(os.path.join(os.path.dirname(__file__), ".."))
-REF = "/root/reference"
 EXDIR = os.path.join(ROOT, "oracle", "_ref", "examples")
-LIBDIR = os.path.join(ROOT, "flac_b200")
+GOLDEN = os.path.join(ROOT, "tests", "golden", "dropin.json")
+# the reference's units the encode client is linked with besides the library (oracle/Makefile, target `examples`)
+METADATA_UNITS = ("metadata_object", "format", "memory", "bitwriter", "stream_encoder_framing", "crc", "bitmath")
 
 LAYOUT_PROBE = r"""
 #include <stddef.h>
@@ -44,38 +46,31 @@ int main(void) {
 """
 
 
-def _have_reference():
-    return os.path.isdir(os.path.join(REF, "include", "FLAC")) and shutil.which("gcc") is not None
+def _golden():
+    with open(GOLDEN) as fh:
+        return json.load(fh)
 
 
-@pytest.mark.skipif(not _have_reference(), reason="/root/reference or gcc not present (GPU box)")
-def test_reference_examples_link_against_libflac_b200(tmp_path):
+def test_reference_examples_link_against_libflac_b200():
+    import flac_b200
     from flac_b200 import build
     build.build()
-    objs = [os.path.join(ROOT, "oracle", "_ref", "obj_default", o + ".o")
-            for o in ("metadata_object", "format", "memory", "bitwriter", "stream_encoder_framing", "crc", "bitmath")]
-    base = ["gcc", "-include", "inttypes.h", f"-I{REF}/include"]
-    link = [f"-L{LIBDIR}", "-lflac_b200", f"-Wl,-rpath,{LIBDIR}", "-lm"]
-    r = subprocess.run(base + [f"{REF}/examples/c/decode/file/main.c", "-o", str(tmp_path / "dec")] + link, capture_output=True, text=True)
-    assert r.returncode == 0, r.stderr
-    if all(os.path.exists(o) for o in objs):
-        r = subprocess.run(base + [f"{REF}/examples/c/encode/file/main.c"] + objs + ["-o", str(tmp_path / "enc")] + link, capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
+    lib = flac_b200.lib()
+    for client, names in _golden()["clients"].items():
+        missing = [n for n in names if not hasattr(lib, n)]
+        assert not missing, f"the reference's {client} example client would not link: {missing} not exported"
 
 
-@pytest.mark.skipif(not _have_reference(), reason="/root/reference or gcc not present (GPU box)")
+@pytest.mark.skipif(shutil.which("gcc") is None, reason="gcc not present")
 def test_struct_layouts_match_reference_headers(tmp_path):
-    outs = []
-    for name, inc, flags in (("ref", '#include "FLAC/all.h"', [f"-I{REF}/include"]),
-                             ("ours", '#include <stdio.h>\n#include "flac_b200_stream.h"', [f"-I{ROOT}/include"])):
-        src = tmp_path / f"layout_{name}.c"
-        src.write_text(LAYOUT_PROBE % inc)
-        exe = tmp_path / f"layout_{name}"
-        r = subprocess.run(["gcc", str(src), "-o", str(exe)] + flags, capture_output=True, text=True)
-        assert r.returncode == 0, r.stderr
-        outs.append(subprocess.run([str(exe)], capture_output=True, text=True).stdout)
-    assert outs[0] == outs[1], "struct layout differs from the reference headers:\n" + "\n".join(
-        f"{a}   |   {b}" for a, b in zip(outs[0].splitlines(), outs[1].splitlines()) if a != b)
+    src = tmp_path / "layout_ours.c"
+    src.write_text(LAYOUT_PROBE % '#include <stdio.h>\n#include "flac_b200_stream.h"')
+    exe = tmp_path / "layout_ours"
+    r = subprocess.run(["gcc", str(src), "-o", str(exe), f"-I{ROOT}/include"], capture_output=True, text=True)
+    assert r.returncode == 0, r.stderr
+    ours, ref = subprocess.run([str(exe)], capture_output=True, text=True).stdout.splitlines(), _golden()["layout"]
+    assert ours == ref, "struct layout differs from the reference headers:\n" + "\n".join(
+        f"{a}   |   {b}" for a, b in zip(ref, ours) if a != b)
 
 
 def _write_wav(path, x):

@@ -6,6 +6,7 @@ import numpy as np
 import pytest
 
 import oraclelib
+import refdata
 import reflib
 import signals
 
@@ -29,11 +30,11 @@ def _gpu_decode(frames, ch, bps, rate, bs, total):
 
 
 def _encoded_frames(x, bps, rate, level, bs=0, source="oracle"):
-    if source == "reference" and reflib.available("default"):
-        _, _, frames = reflib.encode(x, bps, rate=rate, level=level, blocksize=bs, opts=reflib.RefEncOpts(streamable_subset=0))
-        return frames
     enc = oraclelib.Encoder(oraclelib.preset(x.shape[1], bps, rate, level, bs))
-    return enc.encode_stream(x)
+    frames = enc.encode_stream(x)
+    if source == "reference":  # the reference's frames (tests/refdata.py): the oracle's, checked to be exactly those
+        return refdata.encode(x, bps, rate=rate, level=level, blocksize=bs, opts=reflib.RefEncOpts(streamable_subset=0)).frames(witness=frames)
+    return frames
 
 
 @pytest.mark.parametrize("level", range(9))

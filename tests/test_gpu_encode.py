@@ -1,11 +1,13 @@
 """GPU parity tests proper: the CUDA encode path (through the C ABI, host buffers) against
  (1) the CPU restatement oracle/flac_oracle.c, and
- (2) the compiled reference libFLAC (oracle/_ref/*.so) when it travelled to this box,
+ (2) the compiled reference libFLAC (oracle/_ref/*.so), through its answers stored in
+     tests/golden/reference.json.gz (tests/refdata.py),
 frame by frame, bit-exact."""
 import numpy as np
 import pytest
 
 import oraclelib
+import refdata
 import reflib
 import signals
 
@@ -32,15 +34,20 @@ def _assert_same(got, want, what):
     assert not bad, f"{what}: {len(bad)}/{len(want)} frames differ, first {bad[:5]}"
 
 
+def _assert_reference(got, ref, what):
+    """got: frames; ref: the reference's answer (refdata.Encoding)."""
+    assert len(got) == len(ref), f"{what}: frame count {len(got)} != {len(ref)}"
+    bad = ref.mismatches(got)
+    assert not bad, f"{what}: {len(bad)}/{len(ref)} frames differ, first {bad[:5]}"
+
+
 @pytest.mark.parametrize("level", range(9))
 def test_levels_16bit_stereo_vs_oracle_and_reference(level):
     x = signals.music_like(4096 * 10 + 777, 2, 16, 44100, seed=1)
     got = _gpu_frames(x, 16, 44100, level)
     _assert_same(got, _oracle_frames(x, 16, 44100, level), "oracle")
-    if reflib.available("default"):
-        for variant in ("strict", "default"):
-            _, _, ref = reflib.encode(x, 16, rate=44100, level=level, variant=variant)
-            _assert_same(got, ref, f"reference[{variant}]")
+    for variant in ("strict", "default"):
+        _assert_reference(got, refdata.encode(x, 16, rate=44100, level=level, variant=variant), f"reference[{variant}]")
 
 
 @pytest.mark.parametrize("level", [0, 3, 5, 8])
@@ -49,9 +56,7 @@ def test_depths_and_channel_counts(level, ch, bps, rate):
     x = signals.music_like(4096 * 3 + 123, ch, bps, rate, seed=11 + ch)
     got = _gpu_frames(x, bps, rate, level)
     _assert_same(got, _oracle_frames(x, bps, rate, level), "oracle")
-    if reflib.available("default"):
-        _, _, ref = reflib.encode(x, bps, rate=rate, level=level)
-        _assert_same(got, ref, "reference[default]")
+    _assert_reference(got, refdata.encode(x, bps, rate=rate, level=level), "reference[default]")
 
 
 @pytest.mark.parametrize("bs", [16, 17, 32, 33, 192, 256, 576, 1000, 1024, 1152, 2048, 2304, 3072, 4608, 5120, 6144, 8192, 9216])
@@ -86,9 +91,7 @@ def test_stress_inputs(name, level):
     bps = 24 if name.endswith("24") else 16
     got = _gpu_frames(x, bps, 44100, level)
     _assert_same(got, _oracle_frames(x, bps, 44100, level), "oracle")
-    if reflib.available("strict"):
-        _, _, ref = reflib.encode(x, bps, rate=44100, level=level, variant="strict")
-        _assert_same(got, ref, "reference[strict]")
+    _assert_reference(got, refdata.encode(x, bps, rate=44100, level=level, variant="strict"), "reference[strict]")
 
 
 def test_option_matrix():
@@ -131,14 +134,12 @@ def test_multi_launch_chunking_and_frame_numbers():
 def test_reference_decoder_accepts_gpu_stream():
     """flac -t equivalent: the reference decoder decodes our frames (behind a reference-made
     stream header) to the original PCM with no errors."""
-    if not reflib.available("default"):
-        pytest.skip("oracle/_ref not present")
     for ch, bps, level in ((2, 16, 8), (2, 24, 8), (1, 16, 5), (8, 24, 5)):
         x = signals.music_like(4096 * 3 + 50, ch, bps, 48000, seed=31)
-        stream, hdr, _ = reflib.encode(x, bps, rate=48000, level=level)
+        header = refdata.encode(x, bps, rate=48000, level=level, header=True).header
         mine = b"".join(_gpu_frames(x, bps, 48000, level))
-        y, info = reflib.decode(stream[:hdr] + mine, x.shape[0], ch)
-        assert info[3] == 0 and np.array_equal(x, y)
+        y = refdata.decode(header + mine, x.shape[0], ch)
+        assert y.info[3] == 0 and y.matches(x)
 
 
 def test_big_batch_property_round_trip():
@@ -252,9 +253,8 @@ def test_limit_min_bitrate(ch, bps, level, bs):
     plain = _gpu_frames(x, bps, 44100, level, bs)
     if level != 1:  # loose mid-side: the constant frames are coded mid/side only, outside the independent-channel loop
         assert plain != got, "limit_min_bitrate changed nothing"
-    if reflib.available("default"):
-        _, _, ref = reflib.encode(x, bps, rate=44100, level=level, blocksize=bs, opts=reflib.RefEncOpts(limit_min_bitrate=1))
-        _assert_same(got, ref, "reference[default]")
+    ref = refdata.encode(x, bps, rate=44100, level=level, blocksize=bs, opts=reflib.RefEncOpts(limit_min_bitrate=1))
+    _assert_reference(got, ref, "reference[default]")
 
 
 @pytest.mark.parametrize("ch,bps,level,bs,exhaustive", [(2, 16, 5, 0, 0), (2, 16, 8, 0, 0), (2, 24, 5, 0, 0), (1, 16, 3, 0, 0), (2, 16, 5, 1152, 1),
@@ -266,7 +266,5 @@ def test_qlp_coeff_precision_search(ch, bps, level, bs, exhaustive):
     got = _gpu_frames(x, bps, 44100, level, bs, **kw)
     _assert_same(got, _oracle_frames(x, bps, 44100, level, bs, **kw), "oracle")
     assert got != _gpu_frames(x, bps, 44100, level, bs, do_exhaustive_model_search=exhaustive), "precision search changed nothing"
-    if reflib.available("default"):
-        opts = reflib.RefEncOpts(prec_search=1, exhaustive=exhaustive if exhaustive else -1)
-        _, _, ref = reflib.encode(x, bps, rate=44100, level=level, blocksize=bs, opts=opts, variant="strict")
-        _assert_same(got, ref, "reference[strict]")
+    opts = reflib.RefEncOpts(prec_search=1, exhaustive=exhaustive if exhaustive else -1)
+    _assert_reference(got, refdata.encode(x, bps, rate=44100, level=level, blocksize=bs, opts=opts, variant="strict"), "reference[strict]")

@@ -1,5 +1,6 @@
 """Pins oracle/flac_oracle.c (the CPU restatement) against the compiled, unmodified
-reference libFLAC (oracle/_ref/*.so, built by oracle/Makefile from /root/reference).
+reference libFLAC (oracle/_ref/*.so, built by oracle/Makefile), through its answers stored
+in tests/golden/reference.json.gz (tests/refdata.py).
 
 The reference's own tests do not pin encoder bytes (SURVEY.md §0.6: only round trips and
 size monotonicity, test/test_streams.sh:52-79), so encoder parity is pinned by running the
@@ -15,23 +16,21 @@ import numpy as np
 import pytest
 
 import oraclelib
+import refdata
 import reflib
 import signals
-from conftest import require_ref
 
 
 def _frames_equal(x, bps, rate, level, bs=0, variant="strict", opts=None, **cfg_over):
-    _, _, ref_frames = reflib.encode(x, bps, rate=rate, level=level, blocksize=bs, variant=variant, opts=opts)
+    ref = refdata.encode(x, bps, rate=rate, level=level, blocksize=bs, variant=variant, opts=opts)
     enc = oraclelib.Encoder(oraclelib.preset(x.shape[1], bps, rate, level, bs, **cfg_over))
     got = enc.encode_stream(x)
-    assert len(got) == len(ref_frames)
-    bad = [i for i, (a, b) in enumerate(zip(ref_frames, got)) if a != b]
-    return bad, ref_frames, got
+    bad = ref.mismatches(got)
+    return bad, ref, got
 
 
 @pytest.mark.parametrize("level", range(9))
 def test_all_levels_16bit_stereo_both_builds(level):
-    require_ref()
     x = signals.music_like(4096 * 6 + 777, 2, 16, 44100, seed=1)
     for variant in ("strict", "default"):
         bad, _, _ = _frames_equal(x, 16, 44100, level, variant=variant)
@@ -41,7 +40,6 @@ def test_all_levels_16bit_stereo_both_builds(level):
 @pytest.mark.parametrize("level", [0, 3, 5, 8])
 @pytest.mark.parametrize("ch,bps,rate", [(1, 16, 44100), (2, 24, 96000), (8, 24, 192000), (3, 20, 48000), (2, 8, 22050), (1, 12, 8000)])
 def test_depths_and_channel_counts(level, ch, bps, rate):
-    require_ref()
     n = 4096 * 3 + 123
     x = signals.music_like(n, ch, bps, rate, seed=11 + ch)
     for variant in ("strict", "default"):
@@ -52,7 +50,6 @@ def test_depths_and_channel_counts(level, ch, bps, rate):
 @pytest.mark.parametrize("bs", [16, 17, 32, 33, 192, 256, 576, 1000, 1152, 2304, 4608, 8192, 16384])
 @pytest.mark.parametrize("level", [2, 5, 8])
 def test_blocksizes(bs, level):
-    require_ref()
     x = signals.music_like(max(3 * bs + bs // 3, 600), 2, 16, 44100, seed=3)
     opts = reflib.RefEncOpts(streamable_subset=0)
     bad, _, _ = _frames_equal(x, 16, 44100, level, bs=bs, opts=opts)
@@ -77,7 +74,6 @@ STRESS = {
 @pytest.mark.parametrize("name", sorted(STRESS))
 @pytest.mark.parametrize("level", [1, 5, 8])
 def test_stress_inputs(name, level):
-    require_ref()
     x = STRESS[name]()
     bps = 24 if name.endswith("24") else 16
     for variant in ("strict", "default"):
@@ -86,7 +82,6 @@ def test_stress_inputs(name, level):
 
 
 def test_option_matrix():
-    require_ref()
     x = signals.music_like(4096 * 3 + 99, 2, 16, 44100, seed=2)
     cases = [
         (dict(exhaustive=1), dict(do_exhaustive_model_search=1), 5),
@@ -112,7 +107,6 @@ def test_option_matrix():
 def test_tonal_stress_reported_not_gated():
     """G3: pure tones make the LPC normal equations near-singular; the shipped-flags build
     reassociates its FP sums, so only the source-order build is gated."""
-    require_ref()
     x = signals.sine(4096 * 6, 1, 16, 44100, freq=1000.0, freq2=1001.3)
     bad_strict, _, _ = _frames_equal(x, 16, 44100, 8, variant="strict")
     assert bad_strict == []
@@ -125,24 +119,22 @@ def test_tonal_stress_reported_not_gated():
 def test_decoder_round_trip(level, ch, bps):
     """Decoder pin: reference-encoded frames -> oracle decoder == original PCM, and
     oracle-encoded frames -> reference decoder (through a reference-made header) round trip."""
-    require_ref()
     x = signals.music_like(4096 * 2 + 500, ch, bps, 48000, seed=21)
-    stream, hdr, frames = reflib.encode(x, bps, rate=48000, level=level)
-    y = oraclelib.decode_frames(b"".join(frames), ch, bps, 48000, x.shape[0])
+    ref = refdata.encode(x, bps, rate=48000, level=level, header=True)
+    mine = oraclelib.Encoder(oraclelib.preset(ch, bps, 48000, level)).encode_stream(x)
+    y = oraclelib.decode_frames(b"".join(ref.frames(witness=mine)), ch, bps, 48000, x.shape[0])
     assert np.array_equal(x, y)
-    enc = oraclelib.Encoder(oraclelib.preset(ch, bps, 48000, level))
-    mine = b"".join(enc.encode_stream(x))
-    z, info = reflib.decode(stream[:hdr] + mine, x.shape[0], ch)
-    assert info[3] == 0 and np.array_equal(x, z)
+    z = refdata.decode(ref.header + b"".join(mine), x.shape[0], ch)
+    assert z.info[3] == 0 and z.matches(x)
 
 
 def test_decoder_stress_round_trip():
-    require_ref()
     for name in sorted(STRESS):
         x = STRESS[name]()
         bps = 24 if name.endswith("24") else 16
-        _, _, frames = reflib.encode(x, bps, level=8)
-        y = oraclelib.decode_frames(b"".join(frames), x.shape[1], bps, 44100, x.shape[0])
+        ref = refdata.encode(x, bps, level=8)
+        witness = oraclelib.Encoder(oraclelib.preset(x.shape[1], bps, 44100, 8)).encode_stream(x)
+        y = oraclelib.decode_frames(b"".join(ref.frames(witness)), x.shape[1], bps, 44100, x.shape[0])
         assert np.array_equal(x, y), name
 
 
